@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- env-steps/sec (agents x envs x steps / s) of the GCBF+ rollout hot path.
 
-Contract: `python bench.py --gpus N --steps K --warmup W [--impl reference] [--config 3|4|5]`
+Contract: `python bench.py --gpus N --steps K --warmup W [--impl reference] [--config 3|4|5] [--dump-outputs DIR]`
 (N > 1: launched by torch.distributed.run, one rank per GPU).  One JSON line on rank 0.
 
 A "step" is one steady-state T = 256-step closed-loop rollout (SURVEY 8d) of E envs per GPU of a BASELINE.json
@@ -197,6 +197,8 @@ def run_ours(args):
     ms_total = max_over_ranks(ev0.elapsed_time(ev1))
     clocks = sampler.stop() if rank == 0 else {}
     eng.check_overflow()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng.result())
     ms_per_step = ms_total / args.steps
     value = N * E * world * T / (ms_per_step * 1e-3)
 
@@ -267,6 +269,39 @@ def run_ours(args):
         gc.collect()                      # captured graphs holding NCCL kernels must be freed before the communicator
         torch.cuda.synchronize()
         dist.destroy_process_group()
+
+
+DUMP_LIMIT = 63_000_000      # array bytes: with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(out_dir: str, res) -> None:
+    """Writes the last timed rollout as its caller receives it (RolloutEngine.result(), [E, T or T + 1, ...] records) to
+    out_dir/<name>.npy: float32, the per-step edge counts as float64.  Arrays are taken smallest first; each is written
+    whole if it fits in an even share of what is left of DUMP_LIMIT, otherwise as that many of its rows (indices over
+    all axes but the last, which is kept whole), drawn without replacement by one generator of fixed seed -- so the same
+    arguments select the same rows on every run."""
+    import numpy as np
+    import torch
+    outs = {"agent": res.agent, "actions": res.actions, "rewards": res.rewards, "costs": res.costs, "hits": res.hits,
+            "n_edges": res.n_edges.double()}
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(0)
+    left = DUMP_LIMIT
+    order = sorted(outs, key=lambda k: outs[k].numel() * outs[k].element_size())
+    for i, name in enumerate(order):
+        x = outs[name]
+        share = left // (len(order) - i)
+        if x.numel() * x.element_size() <= share:
+            a = x.contiguous().cpu().numpy()
+        else:
+            rows = x.numel() // x.shape[-1]
+            idx = np.sort(rng.choice(rows, share // (x.shape[-1] * x.element_size()), replace=False))
+            sel = tuple(torch.from_numpy(j).to(x.device) for j in np.unravel_index(idx, x.shape[:-1]))
+            a = x[sel].cpu().numpy()
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+        left -= a.nbytes
+        print(f"dump-outputs: {name}.npy {a.dtype} {list(a.shape)}"
+              + ("" if a.shape == tuple(x.shape) else f" (seeded sample of the rows of {list(x.shape)})"), file=sys.stderr)
 
 
 def train_step_bench(torch, dist, env, algo, eng, rank, world, cfg, max_over_ranks, barrier):
@@ -605,7 +640,14 @@ def main():
     ap.add_argument("--no-train", action="store_true")
     ap.add_argument("--train-only", action="store_true",
                     help="profiling aid: one short rollout, then the train-step measurement alone (prints its dict)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last rollout's records (agent, actions, rewards, costs, hits, "
+                         "n_edges) as DIR/<name>.npy, at most 64 MB in all (rank 0's environments)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.train_only):
+        ap.error("--dump-outputs records the rollout of --impl ours and is not available with --train-only")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,6 +1,8 @@
 """CPU: pins the oracle against everything the reference offers for this path (SURVEY 4, 8c):
 LQR gains, parameter trees of the pretrained pickles, closed-form geometry, the
 dense (reference layout) == sparse equivalence, label semantics, optimizer restatement."""
+import hashlib
+import json
 import os
 
 import numpy as np
@@ -36,15 +38,23 @@ def test_pretrained_fixture_counts(env_id, n_actor, n_cbf):
     assert z["cbf:params/GNN_0/GNNLayer_0/update/Dense_0/kernel"].shape == (131, 256)
 
 
-def test_fixture_equals_reference_pickle_when_reference_is_mounted():
-    ref = "/root/reference/pretrained/DoubleIntegrator/gcbf+/models/1000/cbf.pkl"
-    if not os.path.exists(ref):
-        pytest.skip("reference not mounted (GPU box)")
-    from oracle.nn import flatten_params, load_ref_pickle
-    flat = flatten_params(load_ref_pickle(ref))
-    z = np.load(os.path.join(GOLDEN, "params_DoubleIntegrator.npz"))
-    for k, v in flat.items():
-        np.testing.assert_array_equal(z["cbf:" + k], v)
+def test_fixture_equals_reference_pickle():
+    """params_<Env>.npz of every environment holds exactly the leaves of the reference's pretrained {actor,cbf}.pkl:
+    shapes, SHA-256 of the float32 bytes and a seeded sample of values, as recorded from the pickles by
+    tests/golden/make_pickle_digests.py."""
+    g = np.load(os.path.join(GOLDEN, "ref_pickle_digests.npz"))
+    meta = json.loads(str(g["meta"]))
+    assert sorted(meta) == sorted(ENVS)
+    for env_id in ENVS:
+        want = meta[env_id]
+        z = np.load(os.path.join(GOLDEN, f"params_{env_id}.npz"))
+        assert sorted(z.files) == sorted(want), env_id
+        for k, m in want.items():
+            v = z[k]
+            assert v.dtype == np.float32 and list(v.shape) == m["shape"], (env_id, k, v.dtype, v.shape)
+            lo, hi = m["sample"]
+            np.testing.assert_array_equal(v.ravel()[g["index"][lo:hi]], g["value"][lo:hi], err_msg=f"{env_id} {k}")
+            assert hashlib.sha256(np.ascontiguousarray(v).tobytes()).hexdigest() == m["sha256"], (env_id, k)
 
 
 def test_rectangle_raycast_closed_form():
